@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the rewriting_b200 hot path (driver contract).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 metric   : StyleGAN2-256 images/sec (BASELINE.json), synthetic random z, seeded random weights
 workload : SeqStyleGAN2(256, mconv='seq') generator forward, batch=32 per GPU, fp32 in/out,
@@ -24,6 +24,11 @@ roofline : dominant kernel = conv_tc (implicit-GEMM styled conv); achieved = alg
 cpu_baseline / --impl reference: the CPU oracle port of the reference's PyTorch path
            (oracle/sg2_oracle.py; the Python reference itself cannot travel to the GPU box)
            timed on the host cores on a bounded sample (batch 2).
+
+--dump-outputs DIR: after the run, DIR/images.npy holds what the timed path returned in its last
+           step: rank 0's batch of 32 images, float32 [32, 3, 256, 256] (24 MiB).  z and the
+           weights are seeded, so two builds given the same arguments can be compared image
+           for image.
 
 Multi-GPU: one process per GPU under torchrun; z batches are independent (weak scaling, no
 data-path collective for image generation; one all-reduce for the covariance).
@@ -254,7 +259,11 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-graph', action='store_true',
                     help='time eager module calls instead of the CUDA-graph replay')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the images of the last timed step to DIR/images.npy (float32)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         return run_reference(args)
 
@@ -270,7 +279,7 @@ def main():
         os.environ.setdefault('MASTER_ADDR', '127.0.0.1')
         dist.init_process_group('nccl', device_id=device)
     W = max(args.warmup, 3)
-    K = max(args.steps, 1)
+    K = args.steps
 
     from rewriting_b200 import _cabi, ops
     from rewriting_b200.utils import zdataset, nethook, runningstats
@@ -347,6 +356,8 @@ def main():
         e1.record()
         barrier()
         ms_dev = max_over_ranks(e0.elapsed_time(e1))
+        # the graph replay returns its static output buffer, which later replays overwrite
+        last_images = img.float().cpu() if args.dump_outputs and rank == 0 else None
         launches = launches_per_step * K          # a graph replay launches the same kernels
         # per-kernel CUDA-event timing of the dominant kernel: eager replay of the same steps
         # (events cannot be read back from inside a graph), CPU running ahead of the GPU
@@ -524,6 +535,10 @@ def main():
         elif world > 1:
             line['cpu_baseline'] = {'value': None, 'unit': 'images/s', 'cores': os.cpu_count(),
                                     'kind': 'port', 'sample': 'measured at N=1 only'}
+        if last_images is not None:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, 'images.npy'), last_images.numpy())
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -220,13 +220,20 @@ def test_shard_range_partitions_exactly():
             assert max(sizes) - min(sizes) <= 1 and sum(sizes) == n
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/rewrite'),
-                    reason='needs a checkout of the reference (authoring container only)')
-def test_install_aliases_serves_the_reference_ui_over_this_rewriter():
+def test_install_aliases_serves_the_reference_ui_over_this_rewriter(tmp_path):
     """`from rewrite import ganrewrite, rewriteapp` in a notebook: this package's rewriter and
-    overlay renderer, the reference's device-independent GanRewriteApp / widgets."""
+    overlay renderer, the reference's device-independent GanRewriteApp / widgets.  The checkout
+    is a stand-in holding only the module names this package does not provide."""
     import subprocess
     import sys
+    ref = tmp_path / 'reference'
+    for sub, mod, body in (('rewrite', 'rewriteapp', 'class GanRewriteApp(object):\n    pass\n'),
+                           ('rewrite', 'ganrewrite', 'raise ImportError("shadowed")\n'),
+                           ('utils', 'labwidget', 'class Widget(object):\n    pass\n'),
+                           ('utils', 'imgviz', 'raise ImportError("shadowed")\n')):
+        (ref / sub).mkdir(parents=True, exist_ok=True)
+        (ref / sub / '__init__.py').write_text('')
+        (ref / sub / (mod + '.py')).write_text(body)
     code = '''
 import sys, types
 sys.path.insert(0, %r)
@@ -238,15 +245,15 @@ if 'IPython' not in sys.modules:
         d.display = lambda *a, **k: None; m.display = d
         sys.modules['IPython'] = m; sys.modules['IPython.display'] = d
 import rewriting_b200
-rewriting_b200.install_aliases('/root/reference')
+rewriting_b200.install_aliases(%r)
 from rewrite import ganrewrite, rewriteapp
 from utils import imgviz, labwidget, runningstats
 assert ganrewrite.__file__.startswith(%r), ganrewrite.__file__
 assert imgviz.__file__.startswith(%r) and runningstats.__file__.startswith(%r)
-assert rewriteapp.__file__.startswith('/root/reference') and labwidget.__file__.startswith('/root/reference')
+assert rewriteapp.__file__.startswith(%r) and labwidget.__file__.startswith(%r)
 assert hasattr(rewriteapp, 'GanRewriteApp') and hasattr(ganrewrite, 'SeqStyleGanRewriter')
 print('ok')
-''' % (ROOT, ROOT, ROOT, ROOT)
+''' % (ROOT, str(ref), ROOT, ROOT, ROOT, str(ref), str(ref))
     r = subprocess.run([sys.executable, '-W', 'ignore', '-c', code], capture_output=True, text=True,
                        timeout=300)
     assert r.returncode == 0 and r.stdout.strip().endswith('ok'), r.stderr[-2000:]
