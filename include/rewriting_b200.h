@@ -91,8 +91,9 @@ int rw_modconv_up_fwd(const void* kp_hi, const void* kp_lo, const void* wt_hi, c
 /* ---- generation fast path: producers write the consumer's operands directly ----
  * rw_modconv_fwd_fused = rw_modconv_fwd whose epilogue can additionally emit
  *   next_{hi,lo}[rows][Cout] : key planes of the NEXT layer, split_bf16(next_scale[b,o] * y)
- *   rgb_part[Cout/64][B][3][H*W] : this layer's ToRGB partial sums (one per 64-channel group)
- *                                   with rgb_w[B,3,Cout]
+ *   rgb_part[P][B][3][H*W] : this layer's ToRGB partial sums, one per epilogue column group,
+ *                            with rgb_w[B,3,Cout]; P = rw_modconv_rgb_parts(Cout) (Cout/64 for
+ *                            Cout % 128 == 0, 2 for the 64- and 32-channel layers)
  * `out` (fp32 NCHW) becomes optional.  rw_modconv_up_fwd_cl writes the conv_transpose output
  * channels-last per phase, t_cl[4][rows][Cout]; rw_blur_up_fused turns it into the next layer's
  * planes (and/or fp32 NCHW); rw_rgb_combine = sum of partials + bias + 2x-upsampled skip. */
@@ -102,6 +103,9 @@ int rw_modconv_fwd_fused(const void* kp_hi, const void* kp_lo, const void* wt_hi
                          int B, int Cin, int Cout, int H, int W, float* out,
                          const float* next_scale, void* next_hi, void* next_lo,
                          const float* rgb_w, float* rgb_part, rw_stream_t stream);
+/* number of ToRGB partials rw_modconv_fwd_fused writes for Cout output channels; < 1 when the
+ * row-GEMM does not take Cout */
+int rw_modconv_rgb_parts(int Cout);
 int rw_modconv_up_fwd_cl(const void* kp_hi, const void* kp_lo, const void* wt_hi,
                          const void* wt_lo, const float* scale_bo, int B, int Cin, int Cout, int H,
                          int W, float* t_cl, rw_stream_t stream);

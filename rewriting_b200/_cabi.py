@@ -54,6 +54,7 @@ SIGNATURES = {
     'rw_modconv_fwd_fused': (c_int, [c_p, c_p, c_p, c_p, c_p, c_p, c_ll, c_p, c_p, c_int,
                                      c_int, c_int, c_int, c_int, c_int, c_p, c_p, c_p, c_p,
                                      c_p, c_p, c_p]),
+    'rw_modconv_rgb_parts': (c_int, [c_int]),
     'rw_modconv_up_fwd_cl': (c_int, [c_p, c_p, c_p, c_p, c_p, c_int, c_int, c_int, c_int, c_int,
                                      c_p, c_p]),
     'rw_modconv_up_fused': (c_int, [c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_ll, c_p, c_p, c_p, c_p, c_p,

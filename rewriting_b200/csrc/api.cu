@@ -58,7 +58,8 @@ static PFN_encodeTiled get_encode_fn() {
 }
 
 int make_tmap_2d_bf16(CUtensorMap* out, const void* base, uint64_t inner, uint64_t outer,
-                      uint64_t row_stride_bytes, uint32_t box_inner, uint32_t box_outer) {
+                      uint64_t row_stride_bytes, uint32_t box_inner, uint32_t box_outer,
+                      uint32_t swizzle_bytes) {
   PFN_encodeTiled fn = get_encode_fn();
   if (!fn) {
     set_last_error("cuTensorMapEncodeTiled not available from the driver");
@@ -69,12 +70,19 @@ int make_tmap_2d_bf16(CUtensorMap* out, const void* base, uint64_t inner, uint64
                    (unsigned long long)row_stride_bytes);
     return RW_ERR_BAD_ARG;
   }
+  if ((swizzle_bytes != 128 && swizzle_bytes != 64) || box_inner * 2 > swizzle_bytes) {
+    set_last_error("TMA operand: box rows of %u B do not fit a %u B swizzle", box_inner * 2,
+                   swizzle_bytes);
+    return RW_ERR_BAD_ARG;
+  }
   cuuint64_t gdim[2] = {inner, outer};
   cuuint64_t gstr[1] = {row_stride_bytes};
   cuuint32_t box[2] = {box_inner, box_outer};
   cuuint32_t estr[2] = {1, 1};
+  const CUtensorMapSwizzle sw =
+      swizzle_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
   CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), gdim, gstr,
-                  box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                  box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
     set_last_error("cuTensorMapEncodeTiled failed: CUresult %d (inner=%llu outer=%llu box=%ux%u)",
@@ -418,6 +426,8 @@ int rw_modconv_fwd_fused(const void* kp_hi, const void* kp_lo, const void* wt_hi
   return conv_tc_launch(p, kp_hi, kp_lo, wt_hi, wt_lo, 9 * Cin, stream);
 }
 
+int rw_modconv_rgb_parts(int Cout) { return conv_tc_rgb_parts(Cout); }
+
 int rw_modconv_up_fused(const void* kp_hi, const void* kp_lo, const void* wt_hi, const void* wt_lo,
                         const float* demod, const float* kernel4x4, const float* noise,
                         long long noise_bstride, const float* noise_w, const float* bias,
@@ -659,6 +669,11 @@ int rw_conv_wgrad(const void* g_hi, const void* g_lo, const void* kp_hi, const v
     set_last_error("rw_conv_wgrad: bad argument");
     return RW_ERR_BAD_ARG;
   }
+  if (Cout < 128 || Cin < 128 || Cout % 128 != 0 || Cin % 128 != 0) {
+    // the col-GEMM's 128 x 128 tiles: the 64- and 32-channel layers have no weight gradient
+    set_last_error("rw_conv_wgrad: Cout=%d Cin=%d must be multiples of 128", Cout, Cin);
+    return RW_ERR_BAD_ARG;
+  }
   GramTcParams p;
   memset(&p, 0, sizeof(p));
   p.rows = static_cast<int>(rows);
@@ -727,6 +742,11 @@ int rw_conv_up_wgrad(const void* gph_hi, const void* gph_lo, const void* kp_hi, 
   if (!gph_hi || !gph_lo || !kp_hi || !kp_lo || !dw_toi || !workspace || rows <= 0 ||
       rows > 0x7fffffffLL) {
     set_last_error("rw_conv_up_wgrad: bad argument");
+    return RW_ERR_BAD_ARG;
+  }
+  if (Cout < 128 || Cin < 128 || Cout % 128 != 0 || Cin % 128 != 0) {
+    // the col-GEMM's 128 x 128 tiles: the 64- and 32-channel layers have no weight gradient
+    set_last_error("rw_conv_up_wgrad: Cout=%d Cin=%d must be multiples of 128", Cout, Cin);
     return RW_ERR_BAD_ARG;
   }
   GramTcParams p;

@@ -33,7 +33,10 @@ namespace rw {
 namespace {
 
 constexpr int BM = 128;
-constexpr int BK = 64;            // bf16 elements per k-block = one 128B swizzle row
+// BN (N tile = output channels per tile) is 128 for Cout % 128 == 0 and equal to Cout for the
+// 64- and 32-channel tails of the 512^2 / 1024^2 generators (tcgen05 M128 takes N in steps of 16).
+// BK (bf16 elements per k-block) is one swizzle row: 64 = 128 B rows (SWIZZLE_128B) in general,
+// 32 = 64 B rows (SWIZZLE_64B) for Cin = 32.
 constexpr int UMMA_K = 16;
 constexpr int kStages = 3;
 // warp 0 = TMA producer, warp 1 = MMA issuer, warps 2..9 = epilogue: two warps per TMEM lane
@@ -41,7 +44,6 @@ constexpr int kStages = 3;
 // and twice the epilogue throughput for the short-K phase tiles of the upsampling layers)
 constexpr int kNumThreads = 320;
 constexpr int kEpiWarps = 8;
-constexpr int kEpiCols = 64;
 // The tensor core's fp32 accumulate truncates (round-toward-zero) on every MMA: measured
 // relative bias ~ -2^-25 per accumulation (profiles/r1_precision_probe.json), i.e. 1.6e-5
 // after the 864 accumulations of a K=4608 tile.  So a TMEM accumulator only ever holds a
@@ -64,7 +66,7 @@ template <int CG> struct AccGeom {
 // CG = cta_group: 1 = one CTA per 128-row tile; 2 = CTA pair, 256-row tile, each CTA stages its
 // own 128 A rows and HALF of the B (weight) tile -> 25 % less shared-memory traffic per MMA,
 // which is what bounds the 1-CTA kernel (A 4 KB + B 4 KB read per 64-cycle MMA = 125 B/cycle).
-template <int BN, int CG>
+template <int BN, int BK, int CG>
 struct ConvSmem {
   static constexpr int kStagesN = (CG == 2) ? 4 : kStages;
   static constexpr int kABytes = BM * BK * 2;          // one plane
@@ -102,7 +104,10 @@ __device__ __forceinline__ void decode_tile(int tile, int nphase, int nsched, in
 //          mainloop is short, and the generic epilogue's ~37 predicated instructions per column
 //          (2400 per tile and warp) made the MMA issuer wait for TMEM (ncu, layer 13: issuer
 //          spinning on tmem_empty, tensor pipe 52 %).
-template <int BN, int CG, int EPI>
+//
+// Every epilogue warp owns BN / 2 columns of the tile; the ToRGB partials are written per such
+// column group, so a launch writes 2 * Cout / BN of them (conv_tc_rgb_parts).
+template <int BN, int BK, int CG, int EPI>
 __global__ void __launch_bounds__(kNumThreads, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap map_a_hi,
                const __grid_constant__ CUtensorMap map_a_lo,
@@ -111,11 +116,18 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a_hi,
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
                                              ~static_cast<uintptr_t>(1023));
-  using S = ConvSmem<BN, CG>;
+  using S = ConvSmem<BN, BK, CG>;
   constexpr int kSt = S::kStagesN;
   constexpr int kNumAcc = AccGeom<CG>::kNumAcc;
   constexpr int kAccCols = AccGeom<CG>::kAccCols;
-  static_assert(BN == 128, "accumulator geometry assumes 128-column tiles");
+  constexpr int kEpiCols = BN / 2;             // accumulator columns per epilogue warp
+  constexpr int kLdCols = kEpiCols < 32 ? kEpiCols : 32;
+  static_assert(BN == 128 || (CG == 1 && (BN == 64 || BN == 32)), "tile widths: 128, or 64 / 32 single-CTA");
+  static_assert(BK == 64 || BK == 32, "k-block = one 128 B or 64 B swizzle row");
+  static_assert(BN <= kAccCols, "accumulator does not fit its TMEM slot");
+  // smem descriptors: K-major, 8-row swizzle atoms of BK * 2 bytes per row
+  constexpr uint32_t kSwz = (BK == 64) ? kSwizzle128B : kSwizzle64B;
+  constexpr uint32_t kSbo = 8 * BK * 2;
   uint8_t* scratch_base = smem + kSt * S::kStageBytes;
   Barriers* bars = reinterpret_cast<Barriers*>(scratch_base + S::kScratchBytes);
 
@@ -222,11 +234,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a_hi,
             mbar_wait(&bars->full[stage], phase);
             tc_fence_after();
             const uint32_t sa = smem_u32(smem + stage * S::kStageBytes);
-            const uint64_t da_hi = make_smem_desc(sa, 16, 1024, kSwizzle128B);
-            const uint64_t da_lo = make_smem_desc(sa + S::kABytes, 16, 1024, kSwizzle128B);
-            const uint64_t db_hi = make_smem_desc(sa + 2 * S::kABytes, 16, 1024, kSwizzle128B);
-            const uint64_t db_lo =
-                make_smem_desc(sa + 2 * S::kABytes + S::kBBytes, 16, 1024, kSwizzle128B);
+            const uint64_t da_hi = make_smem_desc(sa, 16, kSbo, kSwz);
+            const uint64_t da_lo = make_smem_desc(sa + S::kABytes, 16, kSbo, kSwz);
+            const uint64_t db_hi = make_smem_desc(sa + 2 * S::kABytes, 16, kSbo, kSwz);
+            const uint64_t db_lo = make_smem_desc(sa + 2 * S::kABytes + S::kBBytes, 16, kSbo, kSwz);
             if (elect_one()) {
 #pragma unroll
               for (int kk = 0; kk < BK / UMMA_K; ++kk) {
@@ -258,7 +269,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a_hi,
   } else {
     // ------------------------------ epilogue ----------------------------------
     const int q = warp & 3;                 // TMEM lane quarter this warp may read
-    const int half = (warp - 2) >> 2;       // which 64 of the tile's 128 columns
+    const int half = (warp - 2) >> 2;       // which half of the tile's BN columns
     const int cbase = half * kEpiCols;
     const int img = p.Hp * p.Wp;
     uint8_t* scr = scratch_base + (warp - 2) * 32 * S::kScratchRow;
@@ -272,7 +283,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a_hi,
       const int m0 = (mn / n_tiles) * BM * CG + cta_rank * BM;
       const int prow = m0 + q * 32 + lane;
       const int b = prow / img;
-      const int rem = prow - b * img;
+      const int rem = prow - b * img;       // prow < rows < 2^31; element offsets below are 64-bit
       const int yy = rem / p.Wp;
       const int xx = rem - yy * p.Wp;
       const bool valid = (prow < p.rows) && (yy < Hv) && (xx < Wv);
@@ -287,14 +298,14 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a_hi,
         mbar_wait(&bars->tmem_full[as], aphase);
         tc_fence_after();
 #pragma unroll
-        for (int c0 = 0; c0 < kEpiCols; c0 += 32) {
-          uint32_t v[32];
+        for (int c0 = 0; c0 < kEpiCols; c0 += kLdCols) {
+          uint32_t v[kLdCols];
           const uint32_t taddr = tmem_base + static_cast<uint32_t>(as * kAccCols + cbase + c0) +
                                  (static_cast<uint32_t>(q * 32) << 16);
           tmem_ld_32x32(taddr, v);
           tmem_ld_wait();
 #pragma unroll
-          for (int j = 0; j < 32; ++j) acc[c0 + j] += __uint_as_float(v[j]);
+          for (int j = 0; j < kLdCols; ++j) acc[c0 + j] += __uint_as_float(v[j]);
         }
         tc_fence_before();
         __syncwarp();
@@ -352,7 +363,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a_hi,
           }
         }
         if (rw0) {
-          // one partial per 64-channel group: rgb_part[(n_tile*2 + half)][b][c][y*Wv+x]
+          // one partial per BN/2-channel group: rgb_part[(n_tile*2 + half)][b][c][y*Wv+x]
           const size_t hw = static_cast<size_t>(Hv) * Wv;
           float* rp = p.rgb_part +
                       ((static_cast<size_t>((mn % n_tiles) * 2 + half) * p.B + b) * 3) * hw +
@@ -392,17 +403,22 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a_hi,
         }
       }
       if (EPI == 0 && p.next_hi != nullptr) {
+        // kSeg channels (2 * kSeg bytes of a row) per pass, kSlots 16-byte slots per row
+        constexpr int kSeg = kEpiCols < 32 ? kEpiCols : 32;
+        constexpr int kSlots = kSeg / 8;
+        const int nr0 = lane / kSlots;
+        const int n16 = lane % kSlots;
         const float* ns = p.next_scale + static_cast<size_t>(valid ? b : 0) * p.Cout + n0;
 #pragma unroll
-        for (int part = 0; part < kEpiCols / 32; ++part) {      // 32 channels = 64 B per pass
+        for (int part = 0; part < kEpiCols / kSeg; ++part) {
 #pragma unroll
           for (int plane = 0; plane < 2; ++plane) {
 #pragma unroll
-            for (int j8 = 0; j8 < 4; ++j8) {
+            for (int j8 = 0; j8 < kSlots; ++j8) {
               uint32_t w[4];
 #pragma unroll
               for (int e = 0; e < 4; ++e) {
-                const int j = part * 32 + j8 * 8 + 2 * e;
+                const int j = part * kSeg + j8 * 8 + 2 * e;
                 const float k0 = valid ? __ldg(ns + j) * acc[j] : 0.f;
                 const float k1 = valid ? __ldg(ns + j + 1) * acc[j + 1] : 0.f;
                 const __nv_bfloat162 hh = __floats2bfloat162_rn(k0, k1);
@@ -420,13 +436,13 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a_hi,
             __syncwarp();
             __nv_bfloat16* dstp = static_cast<__nv_bfloat16*>(plane == 0 ? p.next_hi : p.next_lo);
 #pragma unroll
-            for (int it = 0; it < 4; ++it) {
-              const int rr = it * 8 + rr0;
+            for (int it = 0; it < kSlots; ++it) {
+              const int rr = it * (32 / kSlots) + nr0;
               const int grow = m0 + q * 32 + rr;
-              const uint4 v = *reinterpret_cast<const uint4*>(scr + rr * S::kScratchRow + c16 * 16);
+              const uint4 v = *reinterpret_cast<const uint4*>(scr + rr * S::kScratchRow + n16 * 16);
               if (grow < p.rows)
-                *reinterpret_cast<uint4*>(dstp + static_cast<size_t>(grow) * p.Cout + n0 + part * 32 +
-                                          c16 * 8) = v;
+                *reinterpret_cast<uint4*>(dstp + static_cast<size_t>(grow) * p.Cout + n0 + part * kSeg +
+                                          n16 * 8) = v;
             }
             __syncwarp();
           }
@@ -447,25 +463,29 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a_hi,
 
 }  // namespace
 
-template <int CG, int EPI>
+template <int BN, int BK, int CG, int EPI>
 static int conv_tc_launch_cg(const ConvTcParams& p, const void* a_hi, const void* a_lo,
                              const void* w_hi, const void* w_lo, int wk_total,
                              cudaStream_t stream) {
-  constexpr int BN = 128;
+  constexpr uint32_t kSwzBytes = BK * 2;
   CUtensorMap ma_hi, ma_lo, mw_hi, mw_lo;
   int rc;
   const int a_cols = p.a_cols > 0 ? p.a_cols : p.Cin;
-  if ((rc = make_tmap_2d_bf16(&ma_hi, a_hi, a_cols, p.rows, (uint64_t)a_cols * 2, BK, BM))) return rc;
-  if ((rc = make_tmap_2d_bf16(&ma_lo, a_lo, a_cols, p.rows, (uint64_t)a_cols * 2, BK, BM))) return rc;
-  if ((rc = make_tmap_2d_bf16(&mw_hi, w_hi, wk_total, p.Cout, (uint64_t)wk_total * 2, BK, BN / CG)))
+  if ((rc = make_tmap_2d_bf16(&ma_hi, a_hi, a_cols, p.rows, (uint64_t)a_cols * 2, BK, BM, kSwzBytes)))
     return rc;
-  if ((rc = make_tmap_2d_bf16(&mw_lo, w_lo, wk_total, p.Cout, (uint64_t)wk_total * 2, BK, BN / CG)))
+  if ((rc = make_tmap_2d_bf16(&ma_lo, a_lo, a_cols, p.rows, (uint64_t)a_cols * 2, BK, BM, kSwzBytes)))
+    return rc;
+  if ((rc = make_tmap_2d_bf16(&mw_hi, w_hi, wk_total, p.Cout, (uint64_t)wk_total * 2, BK, BN / CG,
+                              kSwzBytes)))
+    return rc;
+  if ((rc = make_tmap_2d_bf16(&mw_lo, w_lo, wk_total, p.Cout, (uint64_t)wk_total * 2, BK, BN / CG,
+                              kSwzBytes)))
     return rc;
 
-  using S = ConvSmem<BN, CG>;
+  using S = ConvSmem<BN, BK, CG>;
   static bool attr_set = false;
   if (!attr_set) {
-    rc = check_cuda(cudaFuncSetAttribute(conv_tc_kernel<BN, CG, EPI>,
+    rc = check_cuda(cudaFuncSetAttribute(conv_tc_kernel<BN, BK, CG, EPI>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, S::kTotal),
                     "conv_tc smem attr");
     if (rc) return rc;
@@ -490,12 +510,35 @@ static int conv_tc_launch_cg(const ConvTcParams& p, const void* a_hi, const void
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   if constexpr (CG == 1) {
-    conv_tc_kernel<BN, 1, EPI><<<sched, kNumThreads, S::kTotal, stream>>>(ma_hi, ma_lo, mw_hi, mw_lo,
-                                                                          p);
+    conv_tc_kernel<BN, BK, 1, EPI><<<sched, kNumThreads, S::kTotal, stream>>>(ma_hi, ma_lo, mw_hi,
+                                                                             mw_lo, p);
     return check_cuda(cudaGetLastError(), "conv_tc launch");
   }
-  return check_cuda(cudaLaunchKernelEx(&cfg, conv_tc_kernel<BN, CG, EPI>, ma_hi, ma_lo, mw_hi, mw_lo, p),
+  return check_cuda(cudaLaunchKernelEx(&cfg, conv_tc_kernel<BN, BK, CG, EPI>, ma_hi, ma_lo, mw_hi, mw_lo,
+                                       p),
                     "conv_tc launch");
+}
+
+// the single-CTA narrow tiles (N = 64 or 32 output channels, k-block 64 or 32 input channels)
+template <int BN, int EPI>
+static int conv_tc_launch_narrow(const ConvTcParams& p, const void* a_hi, const void* a_lo,
+                                 const void* w_hi, const void* w_lo, int wk_total,
+                                 cudaStream_t stream) {
+  if (p.Cin % 64 == 0)
+    return conv_tc_launch_cg<BN, 64, 1, EPI>(p, a_hi, a_lo, w_hi, w_lo, wk_total, stream);
+  return conv_tc_launch_cg<BN, 32, 1, EPI>(p, a_hi, a_lo, w_hi, w_lo, wk_total, stream);
+}
+
+// N tile of a launch with Cout output channels: 128, else 64 / 32 for the narrow layers; 0 = none
+int conv_tc_tile_n(int Cout) {
+  if (Cout > 0 && Cout % 128 == 0) return 128;
+  if (Cout == 64 || Cout == 32) return Cout;
+  return 0;
+}
+
+int conv_tc_rgb_parts(int Cout) {
+  const int bn = conv_tc_tile_n(Cout);
+  return bn ? 2 * (Cout / bn) : 0;
 }
 
 // 0 = automatic (CTA pairs when the launch has at least one full wave of 256-row tiles),
@@ -504,10 +547,13 @@ static int g_conv_cg = -1;
 
 int conv_tc_launch(const ConvTcParams& p, const void* a_hi, const void* a_lo, const void* w_hi,
                    const void* w_lo, int wk_total, cudaStream_t stream) {
-  constexpr int BN = 128;
-  if (p.Cin % BK != 0 || p.Cout % BN != 0 || p.nphase < 1 || p.nphase > 4 || p.rows <= 0) {
-    set_last_error("conv_tc: unsupported shape Cin=%d Cout=%d nphase=%d rows=%d", p.Cin, p.Cout,
-                   p.nphase, p.rows);
+  const int BN = conv_tc_tile_n(p.Cout);
+  // Cin: a multiple of 64 (128 B k-blocks); 32 only for the narrow tiles (64 B k-blocks)
+  const bool cin_ok = p.Cin > 0 && (p.Cin % 64 == 0 || (p.Cin == 32 && BN < 128));
+  if (BN == 0 || !cin_ok || p.nphase < 1 || p.nphase > 4 || p.rows <= 0) {
+    set_last_error("conv_tc: unsupported shape Cin=%d Cout=%d nphase=%d rows=%d (Cout must be a "
+                   "multiple of 128 or 64 / 32, Cin a multiple of 64 or 32 with a narrow Cout)",
+                   p.Cin, p.Cout, p.nphase, p.rows);
     return RW_ERR_BAD_ARG;
   }
   for (int i = 0; i < p.nphase; ++i)
@@ -515,6 +561,17 @@ int conv_tc_launch(const ConvTcParams& p, const void* a_hi, const void* a_lo, co
       set_last_error("conv_tc: phase %d has %d taps", i, p.ph_ntaps[i]);
       return RW_ERR_BAD_ARG;
     }
+  // lean epilogue when only the optional scale and the store are asked for
+  const bool lean = !p.noise && !p.bias && !p.act && !p.rgb_w && !p.rgb_part && !p.next_hi &&
+                    p.out != nullptr && (reinterpret_cast<uintptr_t>(p.scale_bo) & 15u) == 0;
+  if (BN == 64) {
+    if (lean) return conv_tc_launch_narrow<64, 1>(p, a_hi, a_lo, w_hi, w_lo, wk_total, stream);
+    return conv_tc_launch_narrow<64, 0>(p, a_hi, a_lo, w_hi, w_lo, wk_total, stream);
+  }
+  if (BN == 32) {
+    if (lean) return conv_tc_launch_narrow<32, 1>(p, a_hi, a_lo, w_hi, w_lo, wk_total, stream);
+    return conv_tc_launch_narrow<32, 0>(p, a_hi, a_lo, w_hi, w_lo, wk_total, stream);
+  }
   if (g_conv_cg < 0) {
     const char* e = getenv("RW_CONV_CG");
     g_conv_cg = e ? atoi(e) : 0;
@@ -523,18 +580,15 @@ int conv_tc_launch(const ConvTcParams& p, const void* a_hi, const void* a_lo, co
   if (cg != 1 && cg != 2) {
     // CTA pairs (4 stages of 48 KB, 25 % fewer bytes per MMA) for launches with at least one
     // full wave of 256-row tiles; the single-CTA kernel for the small layers
-    const long long tiles256 = ((static_cast<long long>(p.rows) + 255) / 256) * (p.Cout / BN) * p.nphase;
+    const long long tiles256 = ((static_cast<long long>(p.rows) + 255) / 256) * (p.Cout / 128) * p.nphase;
     cg = (tiles256 >= device_sm_count() / 2) ? 2 : 1;
   }
-  // lean epilogue when only the optional scale and the store are asked for
-  const bool lean = !p.noise && !p.bias && !p.act && !p.rgb_w && !p.rgb_part && !p.next_hi &&
-                    p.out != nullptr && (reinterpret_cast<uintptr_t>(p.scale_bo) & 15u) == 0;
   if (cg == 2) {
-    if (lean) return conv_tc_launch_cg<2, 1>(p, a_hi, a_lo, w_hi, w_lo, wk_total, stream);
-    return conv_tc_launch_cg<2, 0>(p, a_hi, a_lo, w_hi, w_lo, wk_total, stream);
+    if (lean) return conv_tc_launch_cg<128, 64, 2, 1>(p, a_hi, a_lo, w_hi, w_lo, wk_total, stream);
+    return conv_tc_launch_cg<128, 64, 2, 0>(p, a_hi, a_lo, w_hi, w_lo, wk_total, stream);
   }
-  if (lean) return conv_tc_launch_cg<1, 1>(p, a_hi, a_lo, w_hi, w_lo, wk_total, stream);
-  return conv_tc_launch_cg<1, 0>(p, a_hi, a_lo, w_hi, w_lo, wk_total, stream);
+  if (lean) return conv_tc_launch_cg<128, 64, 1, 1>(p, a_hi, a_lo, w_hi, w_lo, wk_total, stream);
+  return conv_tc_launch_cg<128, 64, 1, 0>(p, a_hi, a_lo, w_hi, w_lo, wk_total, stream);
 }
 
 }  // namespace rw

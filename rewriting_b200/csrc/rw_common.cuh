@@ -217,6 +217,17 @@ __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, uint32_t (&v)[32])
       : "r"(taddr)
       : "memory");
 }
+// 16-column form for the narrow (BN = 32) tiles
+__device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, uint32_t (&v)[16]) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
+      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n"
+      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]),
+        "=r"(v[7]), "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]),
+        "=r"(v[14]), "=r"(v[15])
+      : "r"(taddr)
+      : "memory");
+}
 __device__ __forceinline__ void tmem_ld_wait() {
   asm volatile("tcgen05.wait::ld.sync.aligned;\n" ::: "memory");
 }
@@ -226,7 +237,7 @@ __device__ __forceinline__ void tmem_ld_wait() {
 // ---------------------------------------------------------------------------
 // Shared-memory matrix descriptor (PTX ISA "tcgen05 matrix descriptor"):
 //  [0,14) start>>4 | [16,30) LBO>>4 | [32,46) SBO>>4 | [46,48) version=1 |
-//  [49,52) base offset | [52] lbo mode | [61,64) swizzle (2 = 128B)
+//  [49,52) base offset | [52] lbo mode | [61,64) swizzle (2 = 128B, 4 = 64B)
 __host__ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr, uint32_t lbo_bytes,
                                                             uint32_t sbo_bytes,
                                                             uint32_t layout_type) {
@@ -239,6 +250,7 @@ __host__ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr, uint
   return d;
 }
 constexpr uint32_t kSwizzle128B = 2;
+constexpr uint32_t kSwizzle64B = 4;
 
 // Instruction descriptor for kind::f16, bf16 x bf16 -> fp32.
 //  [4,6) D fmt (1=f32) | [7,10) A fmt (1=bf16) | [10,13) B fmt | [15] A major
@@ -260,8 +272,10 @@ __device__ __forceinline__ void split_bf16(float x, __nv_bfloat16& hi, __nv_bflo
 // ---------------------------------------------------------------------------
 // host: TMA descriptor encode through the driver entry point (no -lcuda)
 // ---------------------------------------------------------------------------
+// swizzle_bytes: 128 (box rows of 128 B) or 64 (box rows of 64 B)
 int make_tmap_2d_bf16(CUtensorMap* out, const void* base, uint64_t inner, uint64_t outer,
-                      uint64_t row_stride_bytes, uint32_t box_inner, uint32_t box_outer);
+                      uint64_t row_stride_bytes, uint32_t box_inner, uint32_t box_outer,
+                      uint32_t swizzle_bytes = 128);
 
 int device_sm_count();
 

@@ -54,6 +54,10 @@ struct ConvTcParams {
 
 int conv_tc_launch(const ConvTcParams& p, const void* a_hi, const void* a_lo, const void* w_hi,
                    const void* w_lo, int wk_total, cudaStream_t stream);
+// N tile of a Cout-channel launch (128, or 64 / 32 for the narrow layers; 0 = unsupported) and the
+// number of ToRGB partial groups the fused epilogue writes (2 * Cout / N tile)
+int conv_tc_tile_n(int Cout);
+int conv_tc_rgb_parts(int Cout);
 
 // ---------------------------------------------------------------------------
 // fused upsampling StyledConv (upconv_tc.cu): conv_transpose + blur + demod + noise + bias +

@@ -20,17 +20,18 @@ namespace {
 //   -> optional fp32 NCHW copy (the API-visible key) and bf16 hi/lo planes in
 //   the padded-flat layout  [(b, y in 0..H, x in 0..W)][c]  with zero pad row /
 //   pad column.
-// grid: (ceil(Hp*Wp/32), C/64, B), block 256
+// grid: (ceil(Hp*Wp/32), C/CB, B), block 256; CB = 64 channels per block, 32 when C % 64 != 0
 // ---------------------------------------------------------------------------
+template <int CB>
 __global__ void __launch_bounds__(256)
 prep_keys_kernel(const float* __restrict__ x, const float* __restrict__ style, int C, int H, int W,
                  __nv_bfloat16* __restrict__ kp_hi, __nv_bfloat16* __restrict__ kp_lo,
                  float* __restrict__ k_out) {
-  __shared__ float tile[64][33];
+  __shared__ float tile[CB][33];
   const int Hp = H + 1, Wp = W + 1;
   const int img = Hp * Wp;
   const int p0 = blockIdx.x * 32;
-  const int c0 = blockIdx.y * 64;
+  const int c0 = blockIdx.y * CB;
   const int b = blockIdx.z;
   const int t = threadIdx.x;
   {
@@ -39,7 +40,7 @@ prep_keys_kernel(const float* __restrict__ x, const float* __restrict__ style, i
     const int yy = p / Wp, xx = p - yy * Wp;
     const bool valid = (p < img) && (yy < H) && (xx < W);
 #pragma unroll
-    for (int i = 0; i < 8; ++i) {
+    for (int i = 0; i < CB / 8; ++i) {
       const int cl = (t >> 5) + 8 * i;
       float v = 0.f;
       if (valid) {
@@ -53,10 +54,10 @@ prep_keys_kernel(const float* __restrict__ x, const float* __restrict__ style, i
   }
   __syncthreads();
   {
-    const int pl = t >> 3;        // 0..31 position
-    const int cg = (t & 7) * 8;   // 8 channels per thread
+    const int pl = t / (CB / 8);        // position (0..31 used)
+    const int cg = (t % (CB / 8)) * 8;  // 8 channels per thread
     const int p = p0 + pl;
-    if (p < img) {
+    if (pl < 32 && p < img) {
       __align__(16) __nv_bfloat16 h[8];
       __align__(16) __nv_bfloat16 l[8];
 #pragma unroll
@@ -374,32 +375,35 @@ __global__ void add_noise_kernel(const float* __restrict__ x, const float* __res
 //   v = act( FIR4x4(pad(t,1,1)) + noise_w*noise + bias )                       (as blur_up_act)
 //   -> next layer's key planes  split_bf16(next_scale[b,c] * v)  over the padded-flat grid of
 //      the OUTPUT resolution (pad row / column written as zeros), optional fp32 NCHW copy.
-// block: 64 channels x (8 x 16) outputs; thread = (pixel group, channel quad); float4 smem reads.
+// block: 4*QD channels (QD = 16, or 8 when C % 64 != 0) x (8 x 16) outputs, 16*QD threads;
+// thread = (pixel group, channel quad); float4 smem reads.
 // ---------------------------------------------------------------------------
 constexpr int BF_TY = 8, BF_TX = 16, BF_C = 64;
 constexpr int BF_PW = BF_TX + 3, BF_PH = BF_TY + 3;
 
-__global__ void __launch_bounds__(256, 4)
+template <int QD>
+__global__ void __launch_bounds__(16 * QD, 4)
 blur_up_fused_kernel(const float* __restrict__ t_cl, int B, int C, int H, int W,
                      const float* __restrict__ k4, const float* __restrict__ noise,
                      long long noise_bstride, const float* __restrict__ noise_w,
                      const float* __restrict__ bias, int act,
                      const float* __restrict__ next_scale, __nv_bfloat16* __restrict__ next_hi,
                      __nv_bfloat16* __restrict__ next_lo, float* __restrict__ y_out) {
-  extern __shared__ float4 tile4[];      // [BF_PH*BF_PW][16 quads]
+  extern __shared__ float4 tile4[];      // [BF_PH*BF_PW][QD quads]
   __shared__ float kf[16];
+  constexpr int kC = 4 * QD;
   const int Ho = 2 * H, Wo = 2 * W;
   const int Hp_in = H + 1, Wp_in = W + 1;
   const long long rows_in = static_cast<long long>(B) * Hp_in * Wp_in;
-  const int cblocks = C / BF_C;
+  const int cblocks = C / kC;
   const int b = blockIdx.z / cblocks;
-  const int c0 = (blockIdx.z - b * cblocks) * BF_C;
+  const int c0 = (blockIdx.z - b * cblocks) * kC;
   const int ox0 = blockIdx.x * BF_TX, oy0 = blockIdx.y * BF_TY;
   const int tid = threadIdx.x;
   if (tid < 16) kf[tid] = __ldg(k4 + 15 - tid);   // flipped kernel (upfirdn2d correlates)
-  for (int i = tid; i < BF_PH * BF_PW * 16; i += 256) {
-    const int qd = i & 15;
-    const int pos = i >> 4;
+  for (int i = tid; i < BF_PH * BF_PW * QD; i += 16 * QD) {
+    const int qd = i % QD;
+    const int pos = i / QD;
     const int ly = pos / BF_PW, lx = pos - ly * BF_PW;
     const int ty = oy0 + ly - 1, tx = ox0 + lx - 1;
     float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -411,8 +415,8 @@ blur_up_fused_kernel(const float* __restrict__ t_cl, int B, int C, int H, int W,
     tile4[i] = v;
   }
   __syncthreads();
-  const int qd = tid & 15;
-  const int grp = tid >> 4;                 // 16 groups of 8 pixels
+  const int qd = tid % QD;
+  const int grp = tid / QD;                 // 16 groups of 8 pixels
   const int ly = grp >> 1;
   const int lx0 = (grp & 1) * 8;
   const int oy = oy0 + ly;
@@ -434,7 +438,7 @@ blur_up_fused_kernel(const float* __restrict__ t_cl, int B, int C, int H, int W,
   for (int fy = 0; fy < 4; ++fy) {
     float4 tv[11];
 #pragma unroll
-    for (int i = 0; i < 11; ++i) tv[i] = tile4[((ly + fy) * BF_PW + lx0 + i) * 16 + qd];
+    for (int i = 0; i < 11; ++i) tv[i] = tile4[((ly + fy) * BF_PW + lx0 + i) * QD + qd];
 #pragma unroll
     for (int fx = 0; fx < 4; ++fx) {
       const float kk = kf[fy * 4 + fx];
@@ -1177,15 +1181,22 @@ inline int grid_for(long long n, int threads, int cap = 148 * 16) {
 
 int prep_keys_launch(const float* x, const float* style, int B, int C, int H, int W, void* kp_hi,
                      void* kp_lo, float* k_out, cudaStream_t stream) {
-  if (C % 64 != 0) {
-    set_last_error("prep_keys: C=%d must be a multiple of 64", C);
+  if (C % 32 != 0) {
+    set_last_error("prep_keys: C=%d must be a multiple of 32", C);
     return RW_ERR_BAD_ARG;
   }
   const int img = (H + 1) * (W + 1);
-  dim3 grid((img + 31) / 32, C / 64, B);
-  prep_keys_kernel<<<grid, 256, 0, stream>>>(x, style, C, H, W,
-                                             static_cast<__nv_bfloat16*>(kp_hi),
-                                             static_cast<__nv_bfloat16*>(kp_lo), k_out);
+  if (C % 64 == 0) {
+    dim3 grid((img + 31) / 32, C / 64, B);
+    prep_keys_kernel<64><<<grid, 256, 0, stream>>>(x, style, C, H, W,
+                                                   static_cast<__nv_bfloat16*>(kp_hi),
+                                                   static_cast<__nv_bfloat16*>(kp_lo), k_out);
+  } else {
+    dim3 grid((img + 31) / 32, C / 32, B);
+    prep_keys_kernel<32><<<grid, 256, 0, stream>>>(x, style, C, H, W,
+                                                   static_cast<__nv_bfloat16*>(kp_hi),
+                                                   static_cast<__nv_bfloat16*>(kp_lo), k_out);
+  }
   return check_cuda(cudaGetLastError(), "prep_keys launch");
 }
 
@@ -1283,27 +1294,40 @@ int blur_up_fused_launch(const float* t_cl, int B, int C, int Hin, int Win, cons
                          const float* noise, long long noise_bstride, const float* noise_w,
                          const float* bias, int act, const float* next_scale, void* next_hi,
                          void* next_lo, float* y_out, cudaStream_t stream) {
-  if (C % BF_C != 0) {
-    set_last_error("blur_up_fused: C=%d must be a multiple of 64", C);
+  if (C % 32 != 0) {
+    set_last_error("blur_up_fused: C=%d must be a multiple of 32", C);
     return RW_ERR_BAD_ARG;
   }
   const int Ho = 2 * Hin, Wo = 2 * Win;
   const size_t smem = static_cast<size_t>(BF_PH) * BF_PW * 16 * sizeof(float4);
   static bool attr = false;
   if (!attr) {
-    int rc = check_cuda(cudaFuncSetAttribute(blur_up_fused_kernel,
+    int rc = check_cuda(cudaFuncSetAttribute(blur_up_fused_kernel<16>,
                                              cudaFuncAttributeMaxDynamicSharedMemorySize,
                                              static_cast<int>(smem)),
                         "blur_up_fused smem attr");
     if (rc) return rc;
     attr = true;
   }
+  const int tiles_x = (Wo + 1 + BF_TX - 1) / BF_TX, tiles_y = (Ho + 1 + BF_TY - 1) / BF_TY;
+  if (C % BF_C != 0) {
+    // 32-channel multiples: half-width channel blocks on the generic kernel
+    const long long gz32 = static_cast<long long>(B) * (C / 32);
+    if (gz32 > 65535) {
+      set_last_error("blur_up_fused: grid.z %lld too large", gz32);
+      return RW_ERR_BAD_ARG;
+    }
+    dim3 grid(tiles_x, tiles_y, static_cast<unsigned>(gz32));
+    blur_up_fused_kernel<8><<<grid, 128, smem / 2, stream>>>(
+        t_cl, B, C, Hin, Win, k4, noise, noise_bstride, noise_w, bias, act, next_scale,
+        static_cast<__nv_bfloat16*>(next_hi), static_cast<__nv_bfloat16*>(next_lo), y_out);
+    return check_cuda(cudaGetLastError(), "blur_up_fused launch");
+  }
   const long long gz = static_cast<long long>(B) * (C / BF_C);
   if (gz > 65535) {
     set_last_error("blur_up_fused: grid.z %lld too large", gz);
     return RW_ERR_BAD_ARG;
   }
-  const int tiles_x = (Wo + 1 + BF_TX - 1) / BF_TX, tiles_y = (Ho + 1 + BF_TY - 1) / BF_TY;
   const long long ntiles = static_cast<long long>(tiles_x) * tiles_y * gz;
   const long long rows_in4 = 4LL * B * (Hin + 1) * (Win + 1);
   // the generation fast path's configuration runs the pipelined kernel; anything else (no noise,
@@ -1330,7 +1354,7 @@ int blur_up_fused_launch(const float* t_cl, int B, int C, int Hin, int Win, cons
     return check_cuda(cudaGetLastError(), "blur_up_pipe launch");
   }
   dim3 grid(tiles_x, tiles_y, static_cast<unsigned>(gz));
-  blur_up_fused_kernel<<<grid, 256, smem, stream>>>(
+  blur_up_fused_kernel<16><<<grid, 256, smem, stream>>>(
       t_cl, B, C, Hin, Win, k4, noise, noise_bstride, noise_w, bias, act, next_scale,
       static_cast<__nv_bfloat16*>(next_hi), static_cast<__nv_bfloat16*>(next_lo), y_out);
   return check_cuda(cudaGetLastError(), "blur_up_fused launch");

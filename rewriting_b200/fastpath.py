@@ -250,8 +250,9 @@ def _forward(model, z, upto_key_layer, noise_period, out_u8):
                 nh = torch.empty((rows, Cout), dtype=torch.bfloat16, device=dev)
                 nl = torch.empty_like(nh)
             rgb_w = rgb_part = None
-            ntile = Cout // 64          # one ToRGB partial per 64-channel epilogue group
+            ntile = 0
             if rgb is not None:
+                ntile = ops.rgb_parts(Cout)     # one ToRGB partial per epilogue column group
                 rgb_w = rgb_ws[num]                                              # [B,3,Cout]
                 rgb_part = torch.empty((ntile, B, 3, H, W), dtype=torch.float32, device=dev)
             _cabi.call('rw_modconv_fwd_fused', _p(planes.hi), _p(planes.lo), _p(w_hi), _p(w_lo),

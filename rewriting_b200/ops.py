@@ -160,6 +160,14 @@ def weight_planes(weight, kind='fwd', scale=None):
     return val
 
 
+def rgb_parts(Cout):
+    """Number of ToRGB partial sums rw_modconv_fwd_fused writes for a Cout-channel layer."""
+    n = _cabi.load().rw_modconv_rgb_parts(int(Cout))
+    if n < 1:
+        raise _cabi.RwError('the row-GEMM does not take Cout=%d output channels' % Cout)
+    return n
+
+
 def demod_factors(style, wsq, eps=1e-8):
     style = _f32c(style)
     B, Cin = style.shape
